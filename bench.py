@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - MUSIC DOA windows/s on B200 (BASELINE.json metric), one JSON line on stdout.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2] [--impl ours|reference] [--dump-outputs DIR]
   N > 1:  python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path (covariance -> eigenvectors -> pseudospectrum -> peak pick) over one batch of
@@ -47,6 +47,7 @@ from gr_baz_b200.music_doa_helper import calculate_antenna_array_response  # noq
 
 FP64_DFMA_PER_CLK_PER_SM = 64.0  # measured, profiles/r01_microbench.txt (DESIGN.md section 3)
 POOL_WINDOWS = 4096              # distinct synthetic windows behind the large (configs 3-5) streams
+DUMP_BYTES = 64 << 20            # --dump-outputs: at most this much in all
 
 
 def parse():
@@ -62,7 +63,29 @@ def parse():
     ap.add_argument("--no-next-rows", action="store_true", help="skip the planar-input and device-retune legs (SURVEY 8(f) rows)")
     ap.add_argument("--no-other-configs", action="store_true", help="skip BASELINE configs[2..4]")
     ap.add_argument("--nccl-gather", action="store_true", help="N > 1: all-gather the bins with NCCL instead of the fused peer stores (A/B)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0's windows: angles, levels, bins) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_BYTES):
+    """arrays: name -> (W, ...) device tensor.  Angles and levels are written as float32, bins as float64 (exact).  Above
+    `limit` bytes in all, a fixed seeded sample of the windows is written, with its indices as window_index.npy."""
+    host = {k: v.cpu().numpy().astype(np.float64 if k == "bins" else np.float32) for k, v in arrays.items()}
+    W = len(host["bins"])
+    per_window = sum(a[:1].nbytes for a in host.values())
+    if W * per_window > limit:
+        keep = np.sort(np.random.default_rng(0).choice(W, limit // (per_window + 8), replace=False))
+        host = {k: a[keep] for k, a in host.items()}
+        host["window_index"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def workload(cfg_id, windows_override=0):
@@ -657,6 +680,8 @@ def run_ours(args):
     # the gathered bins against the collective they replace (outside the timed region)
     gather_check = None
     last_bins = d_bins2[(stepno[0] - 1) & 1 if (G > 1 and not fused_gather) else 0]
+    if args.dump_outputs and rank == 0:  # before the untimed legs below reuse the output buffers
+        dump_outputs(args.dump_outputs, {"angles": d_ang, "levels": d_lvl, "bins": last_bins})
     if G > 1:
         ref_all = torch.empty((G, W, n), dtype=torch.int32, device=dev)
         dist.all_gather_into_tensor(ref_all.view(-1), last_bins.view(-1))

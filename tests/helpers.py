@@ -1,5 +1,6 @@
 """Shared helpers for the test-suite (oracle-side: allowed to import oracle/)."""
 import glob
+import hashlib
 import os
 
 import numpy as np
@@ -9,6 +10,9 @@ from oracle import music_oracle as mo
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+# what the reference's own work() returned on the test inputs (tests/golden/make_reference_golden.py)
+REFERENCE_GOLDEN = os.path.join(GOLDEN, "reference_source")
+SPECTRUM_SAMPLE = 64  # spectrum bins kept per case besides the peak bins (keeps the fixtures small)
 
 _table_cache = {}
 
@@ -47,3 +51,35 @@ def rel_err(a, b):
     a = np.asarray(a, np.float64)
     b = np.asarray(b, np.float64)
     return float(np.max(np.abs(a - b) / np.abs(b)))
+
+
+def sha256_of(x):
+    return hashlib.sha256(np.ascontiguousarray(x).tobytes()).hexdigest()
+
+
+def case_key(base, over, W):
+    return "c%d_%s_W%d" % (base, "_".join("%s%s" % kv for kv in sorted(over.items())), W)
+
+
+def reference_record(x, K, res):
+    """What a fixture keeps of one reference work_batch() result: angles and levels in full, the spectrum at the peak
+    bins plus a fixed sample of the others (spec_idx), and the hash of the input it was computed from."""
+    peaks = np.rint(np.asarray(res["angles"], np.float64) * K / 360.0).astype(np.int64) % K
+    sample = np.random.default_rng(K).choice(K, min(K, SPECTRUM_SAMPLE), replace=False)
+    idx = np.union1d(sample, peaks.ravel()).astype(np.int32)
+    return {"angles": res["angles"], "levels": res["levels"], "spec_idx": idx, "spectrum": res["spectrum"][:, idx],
+            "in_sha256": np.bytes_(sha256_of(x))}
+
+
+_reference_cache = {}
+
+
+def reference_result(fixture, key, x):
+    """The stored reference result for case `key` of tests/golden/reference_source/<fixture>.npz; `x` must be the input
+    it was recorded from."""
+    if fixture not in _reference_cache:
+        _reference_cache[fixture] = np.load(os.path.join(REFERENCE_GOLDEN, fixture + ".npz"))
+    z = _reference_cache[fixture]
+    rec = {f: z["%s/%s" % (key, f)] for f in ("angles", "levels", "spec_idx", "spectrum", "in_sha256")}
+    assert sha256_of(x) == rec["in_sha256"].item().decode(), "input of case %s differs from the one the fixture was recorded on" % key
+    return rec
