@@ -10,6 +10,7 @@
 // fp64), because P(theta) = 1/||G^H a||^2 is ill-conditioned at the peak (DESIGN.md).
 #pragma once
 #include <cuda_runtime.h>
+#include <math_constants.h>
 #include <stdint.h>
 
 namespace music {
@@ -532,6 +533,12 @@ __device__ __forceinline__ void eig_phase(double v0r, double v0i, double &pr, do
 // (M = 4); otherwise runtime M <= MA with the matrices in local memory.
 // Rw: M x M complex (row-major, interleaved) in global or shared memory; ew (may be null): M
 // ascending eigenvalues; vw: Vt[j][i], eigenvector j contiguous.
+// A covariance with an Inf entry (an Inf input sample) has ||R||_F^2 = Inf, and off <= c * fro holds for off = fro = Inf:
+// without this check the Jacobi loops stop at once and hand out the identity's columns as eigenvectors, i.e. a finite
+// spectrum and a peak.  The reference's eig_sym gets no decomposition there and work() inserts no peak; the solvers
+// therefore return NaN eigenvalues and eigenvectors for any R whose ||R||_F^2 is not finite, as they already did for NaN.
+constexpr double DBL_MAX_FRO = 1.7976931348623157e308;
+
 template <int MA, bool STATIC>
 __device__ __forceinline__ void herm_eig_body(const double *Rw, double *ew, double *vw, const int M)
 {
@@ -573,6 +580,18 @@ __device__ __forceinline__ void herm_eig_body(const double *Rw, double *ew, doub
                     fro += e2;
                     if (i != j) off += e2;
                 }
+        }
+        if (!(fro <= DBL_MAX_FRO)) {  // Inf / NaN in R: no eigenvectors (see DBL_MAX_FRO)
+            if (STATIC) {
+#pragma unroll
+                for (int i = 0; i < MA; ++i)
+#pragma unroll
+                    for (int j = 0; j < MA; ++j) Ar[i][j] = Ai[i][j] = Vr[i][j] = Vi[i][j] = CUDART_NAN;
+            } else {
+                for (int i = 0; i < M; ++i)
+                    for (int j = 0; j < M; ++j) Ar[i][j] = Ai[i][j] = Vr[i][j] = Vi[i][j] = CUDART_NAN;
+            }
+            break;
         }
         if (off <= (M > 4 ? 1e-29 : 1e-32) * fro || off == 0.0) break;  // see eig_coop_kernel for the M > 4 threshold
         if (STATIC && MA == 4) {
@@ -715,6 +734,11 @@ __device__ __forceinline__ void herm_eig4_coop(const double *Rw, double *vw, con
         fro += __shfl_xor_sync(FULL, fro, 1);
         off += __shfl_xor_sync(FULL, off, 2);
         fro += __shfl_xor_sync(FULL, fro, 2);
+        if (live && !(fro <= DBL_MAX_FRO)) {  // Inf / NaN in R, as in herm_eig_body
+#pragma unroll
+            for (int s = 0; s < 4; ++s) ar[s] = ai[s] = vr[s] = vi[s] = CUDART_NAN;
+            live = false;
+        }
         if (off <= 1e-32 * fro || off == 0.0) live = false;  // same test as herm_eig_body (NaN never passes)
         if (!__any_sync(FULL, live)) break;
         eig4_coop_step<1>(ar, ai, vr, vi, j, live);
@@ -791,6 +815,11 @@ __device__ __forceinline__ void eig_coop_warp(double2 *A, double2 *V, double (*r
         fro = warp_sum(fro);
         // rounding keeps the off-diagonal energy of an M x M iterate near 2 M eps^2 ||A||_F^2 (4e-31 at M = 16), so
         // the M = 4 threshold (1e-32) is unreachable here: stop at 1e-29, or when a sweep no longer helps
+        if (!(fro <= DBL_MAX_FRO)) {  // Inf / NaN in R, as in herm_eig_body (fro is the same in every lane)
+            for (int i = lane; i < M * M; i += 32) { A[(i / M) * P + i % M] = make_double2(CUDART_NAN, CUDART_NAN); V[(i / M) * P + i % M] = make_double2(CUDART_NAN, CUDART_NAN); }
+            __syncwarp();
+            break;
+        }
         if (off <= 1e-29 * fro || off == 0.0 || (sweep > 2 && off <= 1e-24 * fro && off >= 0.25 * prev_off)) break;
         prev_off = off;
         for (int step = 0; step < M - 1; ++step) {

@@ -2,7 +2,8 @@
 """Generates tests/golden/reference_source/ - what the reference itself returns on the inputs of the tests that compare
 with it (tests/test_ref_shim.py, tests/test_gpu_zz_reference_source.py, tests/test_boundary_files.py).
 
-  cpu.npz, gpu.npz  per test case: the angles and levels of the reference's own work() (oracle/_ref, built by
+  cpu.npz, gpu.npz, stress.npz
+                    per test case: the angles and levels of the reference's own work() (oracle/_ref, built by
                     oracle/Makefile target `ref`), its spectrum at the peak bins plus a fixed sample of the others, and the
                     sha256 of the regenerated input (helpers.reference_record).
   surface.json      the signature of the reference's grc/baz_music_doa.xml and the declarations of its
@@ -23,6 +24,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import helpers  # noqa: E402
+import stress_inputs  # noqa: E402
 import test_boundary_files as tb  # noqa: E402
 import test_gpu_zz_reference_source as tg  # noqa: E402
 import test_ref_shim as tr  # noqa: E402
@@ -65,6 +67,14 @@ def gpu_fixture():
     return d
 
 
+def stress_fixture():
+    d = {}
+    for key in stress_inputs.CASES:
+        cfg, table, x = stress_inputs.case(key)
+        record(d, key, x, cfg["m"], cfg["n"], cfg["resolution"], table)
+    return d
+
+
 def surface(reference_dir):
     grc = ET.parse(os.path.join(reference_dir, "grc", "baz_music_doa.xml")).getroot()
     with open(os.path.join(reference_dir, "lib", "baz_music_doa.h")) as f:
@@ -79,7 +89,7 @@ def main():
     if not ref_build.available():
         raise SystemExit("oracle/_ref is not built (oracle/Makefile target `ref`)")
     os.makedirs(helpers.REFERENCE_GOLDEN, exist_ok=True)
-    for name, d in (("cpu", cpu_fixture()), ("gpu", gpu_fixture())):
+    for name, d in (("cpu", cpu_fixture()), ("gpu", gpu_fixture()), ("stress", stress_fixture())):
         np.savez_compressed(os.path.join(helpers.REFERENCE_GOLDEN, name + ".npz"), **d)
     with open(os.path.join(helpers.REFERENCE_GOLDEN, "surface.json"), "w") as f:
         json.dump(surface(sys.argv[1]), f, indent=1)
