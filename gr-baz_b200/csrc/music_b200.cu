@@ -45,9 +45,11 @@ struct DeviceTable {
 struct Workspace {
     double *R = nullptr, *ev = nullptr, *Vt = nullptr, *P64 = nullptr;
     uint32_t cap = 0, p64_cap = 0;
-    cudaEvent_t cov_done = nullptr, scan_done = nullptr;
+    cudaEvent_t scan_done = nullptr;
     bool used = false;
 };
+
+constexpr int NSLOT = 2;  // workspace slots: one per host staging stream (process_device on a caller stream shares slot 0)
 
 }  // namespace
 
@@ -70,29 +72,19 @@ struct music_b200 {
     uint32_t peak_excl = 0;
     unsigned steer_guarded = 0;    // entries of the last built table re-evaluated with the host libm
 
-    // fp64 workspace slots (R, eigenvalues, sorted eigenvectors, optional strengths) and the two
-    // internal streams of the cov -> eig/scan pipeline
-    Workspace ws[3];
-    cudaStream_t s_cov = nullptr, s_scan = nullptr;
-    cudaEvent_t ev_in = nullptr;
-    bool pipeline = false;   // MUSIC_B200_PIPE=1 enables the sub-batch pipeline (launch-bound at 10k windows: off)
+    // fp64 workspace slots (R, eigenvalues, sorted eigenvectors, optional strengths) of the three-kernel path
+    Workspace ws[NSLOT];
     unsigned *work_ctr = nullptr;      // persistent kernels: ring of self-resetting (window tickets, finished CTAs) pairs, CTR_RING per slot
     unsigned ctr_seq[2] = {0, 0};      // next ring entry per slot
     bool fused_spec = true;            // the spectrum port on the fused M = 4 kernel (MUSIC_B200_FUSED_SPEC=0: three-kernel path)
-    int early_drain = 0;               // fused kernel: drain beside the last tensor-core passes (MUSIC_B200_EARLY_DRAIN)
-    int drain_nch = 16;                // fused kernel: drain units per group (MUSIC_B200_DRAIN_NCH, 1..32)
-    unsigned idle_ns = 100;            // fused kernel: sleep of an idle drain worker (MUSIC_B200_IDLE_NS)
     bool pdl = true;                   // fused M = 4 kernel: programmatic dependent launch (MUSIC_B200_PDL=0 turns it off)
     cudaEvent_t fused_done = nullptr;  // orders persistent launches that share a ticket counter but not a stream
     bool fused_used[2] = {false, false};
-    int eig_mode = 0;                 // fused kernel: 0 principal eigenvector by squaring (default), 1 / 2 Jacobi with four lanes / one lane per window (MUSIC_B200_EIG=jacobi|jacobi1)
+    bool eig_mode = false;            // fused kernels: false principal eigenvector by squaring (default), true Jacobi for every window (MUSIC_B200_EIG=jacobi)
     unsigned *f8_stats = nullptr;     // fused M = 8 kernel: windows solved by squaring / by the Jacobi fallback
     int mma_fin_max = 3;              // fused kernel: no tensor-core pass starts once the tickets have run out and this many covariance warps are done (MUSIC_B200_MMA_FIN; 0: at ticket exhaustion, -1: fp64 drain only)
     long long *fused_trace = nullptr;  // MUSIC_B200_TRACE=1: per-CTA clock64 trace of the fused kernel (tools/fused_trace.py)
     bool fused = true;       // MUSIC_B200_FUSED=0 forces the three-kernel path
-    bool covn = true;        // MUSIC_B200_COVN=0: M = 8/16 covariance by the v1 LDG tile kernels
-    bool scan_fast = true;   // MUSIC_B200_SCAN=general disables the specialised n == 1 kernel
-    int cov_tma_stages = 6;  // 0 = LDG tile kernel (MUSIC_B200_COV=ldg), 4 or 6 = TMA ring depth
     // optional per-stage timing (bench.py's roofline leg): events around K1/K2/K3/top-n per chunk
     bool timing = false;
     std::vector<cudaEvent_t> tev;   // 5 events per timed chunk
@@ -210,8 +202,6 @@ int build_table(music_b200 *h, int slot, const double *pos_xy, double lambda, cu
     CU(h, cudaMemcpyAsync(&cnt, h->steer_count, sizeof(unsigned), cudaMemcpyDeviceToHost, st));
     CU(h, cudaStreamSynchronize(st));
     h->steer_guarded = cnt;
-    static const bool no_guard = getenv("MUSIC_B200_STEER_NOGUARD") != nullptr;  // diagnostics: raw device table
-    if (no_guard) return finish_table(h, slot, st);
     if (cnt > (unsigned)STEER_GUARD_CAP) {
         // more boundary cases than the list holds (a degenerate geometry, e.g. all elements at the origin, makes
         // every entry exactly (1, 0)): evaluate every entry the literal way
@@ -253,6 +243,21 @@ EncodeTiledFn encode_tiled_fn()
     return fn;
 }
 
+// 3-D tensor map over the M-antenna input d_in viewed as rows of 128 bytes (16 / M snapshots each; with SWIZZLE_128B a
+// narrower inner box would be padded to the 128-byte span): {32 floats, N * M / 16 rows, W windows}, box {32, box_rows, 1}.
+// False when the driver cannot encode it.
+bool encode_row_map(CUtensorMap *tm, const float *d_in, int M, int N, uint32_t W, int box_rows)
+{
+    const EncodeTiledFn enc = encode_tiled_fn();
+    if (!enc) return false;
+    const cuuint64_t gdim[3] = {32u, (cuuint64_t)(N / (16 / M)), (cuuint64_t)W};
+    const cuuint64_t gstr[2] = {128u, (cuuint64_t)(8 * M) * (cuuint64_t)N};
+    const cuuint32_t box[3] = {32u, (cuuint32_t)box_rows, 1u};
+    const cuuint32_t estr[3] = {1u, 1u, 1u};
+    return enc(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float *>(d_in), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+               CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
 // Inside the chunk loops of the host entry points an error must not skip the common tail (stream syncs, slot
 // reset): record it in rc and leave the loop instead of returning.
 #define CU_BREAK(h, rc, expr)                                                                    \
@@ -266,8 +271,6 @@ EncodeTiledFn encode_tiled_fn()
     }
 
 constexpr unsigned CTR_RING = 256;  // ticket-counter pairs per slot (see ticket_counter)
-constexpr int NSLOT = 3;           // workspace ring for the cov -> eig/scan software pipeline
-constexpr uint32_t MIN_SUB = 1024; // windows; below 2*MIN_SUB a call is not split
 
 // Windows per sub-batch bounding one workspace slot to ~384 MiB.
 uint32_t max_sub_windows(const music_b200 *h, bool need_p64)
@@ -310,7 +313,9 @@ void launch_scan(music_b200 *h, const Workspace &ws, const double *soa, uint32_t
     if (argmax == A && p64 == P && spec == S)                                                           \
         scan_kernel<MT, A, P, S><<<grid, TILE, smem, st>>>(soa, ws.Vt, (int)h->m, (int)h->n, (int)h->K,  \
                                                            (int)W, po, d_spec, d_p64);
-    SCAN_CASE(true, false, false)
+    if constexpr (MT == 0) {  // (M = 4, 8, 16 take scan_peak1_kernel for this case)
+        SCAN_CASE(true, false, false)
+    }
     SCAN_CASE(true, false, true)
     SCAN_CASE(true, true, false)
     SCAN_CASE(true, true, true)
@@ -362,42 +367,22 @@ unsigned *ticket_counter(music_b200 *h, int slot, cudaStream_t st)
 void launch_cov(music_b200 *h, const Workspace &ws, const float *d_in, uint32_t W, cudaStream_t st, int ctr_slot)
 {
     const int M = (int)h->m, N = (int)h->N;
-    if (M == 4 && h->cov_tma_stages > 0) {
+    CUtensorMap tm;
+    if (M == 4) {
         // persistent, one CTA per SM, per-warp TMA ring (see cov4_tma_kernel)
-        const int stages = h->cov_tma_stages;
-        const size_t smem = 1024 + (size_t)COV_WARPS * stages * COV_CHUNK;
         const int grid = std::min<int>(h->sm_count, (int)((W + COV_WARPS - 1) / COV_WARPS));
-        if (stages == 6) cov4_tma_kernel<6><<<grid, COV_WARPS * 32, smem, st>>>(d_in, ws.R, (int)W, N);
-        else cov4_tma_kernel<4><<<grid, COV_WARPS * 32, smem, st>>>(d_in, ws.R, (int)W, N);
+        cov4_tma_kernel<<<grid, COV_WARPS * 32, COV_SMEM, st>>>(d_in, ws.R, (int)W, N);
         h->launches++;
-    } else if ((M == 8 || M == 16) && h->covn && N >= 128 && N % (16 / M) == 0 && encode_tiled_fn()) {
-        // TMA-tiled, window staged once per group of warps (music_covn.cuh)
-        CUtensorMap tm;
-        // rows of 128 bytes (SPR snapshots each): with SWIZZLE_128B a narrower inner box would be padded to the span
-        const int SPR = 16 / M;  // snapshots per 128-byte row
-        const cuuint64_t gdim[3] = {32u, (cuuint64_t)(N / SPR), (cuuint64_t)W};
-        const cuuint64_t gstr[2] = {128u, (cuuint64_t)(8 * M) * (cuuint64_t)N};
-        const cuuint32_t box[3] = {32u, (cuuint32_t)(M == 8 ? 32 * CovNJobs<8>::STEPS * 8 * 8 / 128 : 32 * CovNJobs<16>::STEPS * 8 * 16 / 128), 1u};  // one stage
-        const cuuint32_t estr[3] = {1u, 1u, 1u};
-        const CUresult cr = encode_tiled_fn()(&tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float *>(d_in), gdim, gstr, box, estr,
-                                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                              CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (cr == CUDA_SUCCESS) {
-            constexpr int groups8 = CN_WARPS / CovNJobs<8>::J, groups16 = CN_WARPS / CovNJobs<16>::J;
-            const int groups = M == 8 ? groups8 : groups16;
-            const int grid = std::min<int>(h->sm_count, (int)((W + groups - 1) / groups));
-            unsigned *ctr = ticket_counter(h, ctr_slot, st);
-            if (M == 8) covN_tma_kernel<8><<<grid, CN_WARPS * 32, CN_SMEM, st>>>(tm, ws.R, (int)W, N, ctr);
-            else covN_tma_kernel<16><<<grid, CN_WARPS * 32, CN_SMEM, st>>>(tm, ws.R, (int)W, N, ctr);
-            h->launches++;
-            return;
-        }
-        // (encode failed: fall through is not possible inside this else-if chain; use the tile kernels)
-        const int T = M / 4;
-        const int wpb = 8;
-        cov_tile_kernel<false><<<(unsigned)(((long long)W * T + wpb - 1) / wpb), wpb * 32, 0, st>>>(d_in, ws.R, (int)W, N, M);
-        cov_tile_kernel<true><<<(unsigned)(((long long)W * (T * (T - 1) / 2) + wpb - 1) / wpb), wpb * 32, 0, st>>>(d_in, ws.R, (int)W, N, M);
-        h->launches += 2;
+    } else if ((M == 8 || M == 16) && N >= 128 && N % (16 / M) == 0 &&
+               encode_row_map(&tm, d_in, M, N, W, M == 8 ? 32 * CovNJobs<8>::STEPS * 8 * 8 / 128 : 32 * CovNJobs<16>::STEPS * 8 * 16 / 128)) {
+        // TMA-tiled, window staged once per group of warps (music_covn.cuh); the box is one stage
+        constexpr int groups8 = CN_WARPS / CovNJobs<8>::J, groups16 = CN_WARPS / CovNJobs<16>::J;
+        const int groups = M == 8 ? groups8 : groups16;
+        const int grid = std::min<int>(h->sm_count, (int)((W + groups - 1) / groups));
+        unsigned *ctr = ticket_counter(h, ctr_slot, st);
+        if (M == 8) covN_tma_kernel<8><<<grid, CN_WARPS * 32, CN_SMEM, st>>>(tm, ws.R, (int)W, N, ctr);
+        else covN_tma_kernel<16><<<grid, CN_WARPS * 32, CN_SMEM, st>>>(tm, ws.R, (int)W, N, ctr);
+        h->launches++;
     } else if (M % 4 == 0) {
         const int T = M / 4;
         const int wpb = 8;
@@ -487,7 +472,7 @@ int launch_eig_scan(music_b200 *h, const Workspace &ws, uint32_t W, const PeakOu
     const bool argmax = (h->n == 1) && !local;
     const bool need_p64 = !argmax || d_P64_out != nullptr;
     double *p64 = d_P64_out ? d_P64_out : ws.P64;
-    const bool fast = argmax && !need_p64 && !d_spec && (M == 4 || M == 8 || M == 16) && h->scan_fast;
+    const bool fast = argmax && !need_p64 && !d_spec && (M == 4 || M == 8 || M == 16);
     if (fast) {
         const int grid = (W + SCAN_B - 1) / SCAN_B;
         if (M == 4) scan_peak1_kernel<4><<<grid, TILE, 0, st>>>(soa, ws.Vt, (int)h->K, (int)W, po);
@@ -517,11 +502,6 @@ int launch_eig_scan(music_b200 *h, const Workspace &ws, uint32_t W, const PeakOu
     return MUSIC_B200_OK;
 }
 
-// Enqueue `nwindows` windows.  Large calls are cut into sub-batches and software-pipelined over
-// two internal streams: K1 (HBM-bound, FP64 pipe ~1/3 busy) of sub-batch j+1 runs concurrently
-// with K2+K3 (FP64-only) of sub-batch j, each sub-batch owning one workspace slot.  `st` is
-// ordered before the first and after the last piece of work.  Small calls, and calls made while
-// stage timing is on, run serially on `st`.
 // K1 on planar streams (music_planar.cuh): windows first .. first + W - 1 of the call
 void launch_cov_planar(music_b200 *h, const Workspace &ws, const PlanarStreams &S, unsigned long long first_snapshot,
                        unsigned hop, uint32_t W, cudaStream_t st)
@@ -536,9 +516,12 @@ void launch_cov_planar(music_b200 *h, const Workspace &ws, const PlanarStreams &
     }
 }
 
+// Enqueue `nwindows` windows on `st`: one persistent launch where a fused kernel covers the call, otherwise the three-kernel
+// path in sub-batches of at most max_sub_windows() windows through workspace slot `slot`.  `slot` (0 / 1) also picks the
+// ticket-counter ring of the persistent kernels.
 int enqueue_device(music_b200 *h, const float *d_in, uint32_t nwindows, float *d_ang, float *d_lvl, float *d_spec,
-                   int32_t *d_bins, double *d_P64, double *d_R, double *d_ev, cudaStream_t st, int first_slot,
-                   bool allow_pipeline, const PlanarStreams *planar = nullptr, unsigned hop = 0)
+                   int32_t *d_bins, double *d_P64, double *d_R, double *d_ev, cudaStream_t st, int slot,
+                   const PlanarStreams *planar = nullptr, unsigned hop = 0)
 {
     if (nwindows == 0) return MUSIC_B200_OK;
     if ((!planar && !d_in) || !d_ang) return fail(h, MUSIC_B200_EINVAL, "d_in_c64 and d_angles must not be NULL");
@@ -555,7 +538,7 @@ int enqueue_device(music_b200 *h, const float *d_in, uint32_t nwindows, float *d
         cudaEvent_t *tev = timing_events(h);
         if (tev) cudaEventRecord(tev[0], st);
         const int grid = std::min<int>(h->sm_count, (int)((nwindows + FZ_COV_WARPS - 1) / FZ_COV_WARPS));
-        unsigned *ctr = ticket_counter(h, first_slot, st);
+        unsigned *ctr = ticket_counter(h, slot, st);
         const DeviceTable &tb = h->table[h->cur_table];
         const PeakOut po = make_peak_out(h, d_ang, d_lvl, d_bins, 0);
         const GatherFlags gf = make_gather_flags(h, true);
@@ -571,17 +554,18 @@ int enqueue_device(music_b200 *h, const float *d_in, uint32_t nwindows, float *d
         lc.attrs = la; lc.numAttrs = h->pdl ? 1 : 0;
         const int W_i = (int)nwindows, N_i = (int)h->N, K_i = (int)h->K;
         const bool tr = h->fused_trace != nullptr;  // MUSIC_B200_TRACE=1: the instantiation with the clock64 trace
+        // drain workers: 100 ns idle sleep, 16 chunks per group, no early drain (DESIGN.md section 5)
         const unsigned char *fz = tb.fz;
         const float *c64 = tb.c64, *na_max = tb.na_max;
         cudaError_t le;
         if (planar) {
             auto kern = tr ? music4_fused_kernel<true, true> : music4_fused_kernel<true, false>;
             le = cudaLaunchKernelEx(&lc, kern, (const float *)nullptr, *planar, 0ull, (unsigned)hop, fz, c64, na_max, W_i, N_i, K_i, po, ctr,
-                                    h->fused_trace, h->eig_mode, gf, h->mma_fin_max, h->idle_ns, h->drain_nch, h->early_drain, d_spec);
+                                    h->fused_trace, (int)h->eig_mode, gf, h->mma_fin_max, 100u, 16, 0, d_spec);
         } else {
             auto kern = tr ? music4_fused_kernel<false, true> : music4_fused_kernel<false, false>;
             le = cudaLaunchKernelEx(&lc, kern, d_in, PlanarStreams{}, 0ull, 0u, fz, c64, na_max, W_i, N_i, K_i, po, ctr, h->fused_trace,
-                                    h->eig_mode, gf, h->mma_fin_max, h->idle_ns, h->drain_nch, h->early_drain, d_spec);
+                                    (int)h->eig_mode, gf, h->mma_fin_max, 100u, 16, 0, d_spec);
         }
         CU(h, le);
         h->launches++;
@@ -589,74 +573,45 @@ int enqueue_device(music_b200 *h, const float *d_in, uint32_t nwindows, float *d
         CU(h, cudaGetLastError());
         return MUSIC_B200_OK;
     }
+    CUtensorMap tm;
     if (!planar && h->fused && !local_peaks && h->m == 8 && h->n == 1 && !d_spec && !d_P64 && !d_R && !d_ev && h->N >= 128 &&
-        h->N % 2 == 0 && encode_tiled_fn()) {
+        h->N % 2 == 0 && encode_row_map(&tm, d_in, 8, (int)h->N, nwindows, F8_STAGE / 128)) {
         // M = 8: whole call in one persistent launch (music_fused8.cuh); R and the eigenvectors stay in shared memory
-        CUtensorMap tm;
-        const cuuint64_t gdim[3] = {32u, (cuuint64_t)(h->N / 2), (cuuint64_t)nwindows};  // 128-byte rows of two snapshots
-        const cuuint64_t gstr[2] = {128u, (cuuint64_t)64 * (cuuint64_t)h->N};
-        const cuuint32_t box[3] = {32u, (cuuint32_t)(F8_STAGE / 128), 1u};
-        const cuuint32_t estr[3] = {1u, 1u, 1u};
-        if (encode_tiled_fn()(&tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float *>(d_in), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS) {
-            cudaEvent_t *tev = timing_events(h);
-            if (tev) cudaEventRecord(tev[0], st);
-            const int grid = std::min<int>(h->sm_count, (int)((nwindows + F8_WARPS - 1) / F8_WARPS));
-            unsigned *ctr = ticket_counter(h, first_slot, st);
-            music8_fused_kernel<<<grid, F8_WARPS * 32, F8_SMEM, st>>>(tm, h->table[h->cur_table].soa, (int)nwindows, (int)h->N, (int)h->K,
-                                                                     make_peak_out(h, d_ang, d_lvl, d_bins, 0), ctr, make_gather_flags(h, true),
-                                                                     h->eig_mode ? 1 : 0, h->f8_stats);
-            h->launches++;
-            if (tev) for (int i = 1; i < 5; ++i) cudaEventRecord(tev[i], st);
-            CU(h, cudaGetLastError());
-            return MUSIC_B200_OK;
-        }
+        cudaEvent_t *tev = timing_events(h);
+        if (tev) cudaEventRecord(tev[0], st);
+        const int grid = std::min<int>(h->sm_count, (int)((nwindows + F8_WARPS - 1) / F8_WARPS));
+        unsigned *ctr = ticket_counter(h, slot, st);
+        music8_fused_kernel<<<grid, F8_WARPS * 32, F8_SMEM, st>>>(tm, h->table[h->cur_table].soa, (int)nwindows, (int)h->N, (int)h->K,
+                                                                 make_peak_out(h, d_ang, d_lvl, d_bins, 0), ctr, make_gather_flags(h, true),
+                                                                 h->eig_mode, h->f8_stats);
+        h->launches++;
+        if (tev) for (int i = 1; i < 5; ++i) cudaEventRecord(tev[i], st);
+        CU(h, cudaGetLastError());
+        return MUSIC_B200_OK;
     }
     const bool internal_p64 = (h->n != 1 || local_peaks) && !d_P64;
-    const uint32_t max_sub = max_sub_windows(h, internal_p64);
-    const bool pipe = allow_pipeline && h->pipeline && !h->timing && nwindows >= 2 * MIN_SUB;
-    uint32_t sub;
-    if (pipe) {
-        const uint32_t nsub = std::min<uint32_t>(8, std::max<uint32_t>(2, nwindows / MIN_SUB));
-        sub = ((nwindows + nsub - 1) / nsub + SCAN_B - 1) / SCAN_B * SCAN_B;
-        sub = std::min(sub, max_sub);
-    } else {
-        sub = std::min((nwindows + SCAN_B - 1) / SCAN_B * SCAN_B, max_sub);
-    }
-    cudaStream_t s_cov = pipe ? h->s_cov : st, s_scan = pipe ? h->s_scan : st;
-    if (pipe) {
-        CU(h, cudaEventRecord(h->ev_in, st));
-        CU(h, cudaStreamWaitEvent(s_cov, h->ev_in, 0));
-    }
-    int slot = first_slot, last_slot = -1;
+    const uint32_t sub = std::min((nwindows + SCAN_B - 1) / SCAN_B * SCAN_B, max_sub_windows(h, internal_p64));
+    Workspace &ws = h->ws[slot];
+    int rc = ensure_slot(h, ws, sub, internal_p64);
+    if (rc) return rc;
+    if (ws.used) CU(h, cudaStreamWaitEvent(st, ws.scan_done, 0));  // the slot's last user may be another stream
     for (uint32_t w0 = 0; w0 < nwindows; w0 += sub) {
         const uint32_t W = std::min(sub, nwindows - w0);
-        Workspace &ws = h->ws[slot];
-        int rc = ensure_slot(h, ws, sub, internal_p64);
-        if (rc) return rc;
-        if (ws.used) CU(h, cudaStreamWaitEvent(s_cov, ws.scan_done, 0));  // slot free again
         cudaEvent_t *tev = timing_events(h);
-        if (tev) cudaEventRecord(tev[0], s_cov);
-        if (planar) launch_cov_planar(h, ws, *planar, (unsigned long long)w0 * hop, hop, W, s_cov);
-        else launch_cov(h, ws, d_in + (size_t)w0 * h->nsamples * 2, W, s_cov, first_slot);
-        if (tev) cudaEventRecord(tev[1], s_cov);
-        if (pipe) {
-            CU(h, cudaEventRecord(ws.cov_done, s_cov));
-            CU(h, cudaStreamWaitEvent(s_scan, ws.cov_done, 0));
-        }
+        if (tev) cudaEventRecord(tev[0], st);
+        if (planar) launch_cov_planar(h, ws, *planar, (unsigned long long)w0 * hop, hop, W, st);
+        else launch_cov(h, ws, d_in + (size_t)w0 * h->nsamples * 2, W, st, slot);
+        if (tev) cudaEventRecord(tev[1], st);
         rc = launch_eig_scan(h, ws, W,
                              make_peak_out(h, d_ang + (size_t)w0 * h->n, d_lvl ? d_lvl + (size_t)w0 * h->n : nullptr,
                                            d_bins ? d_bins + (size_t)w0 * h->n : nullptr, w0),
                              d_spec ? d_spec + (size_t)w0 * h->K : nullptr,
                              d_P64 ? d_P64 + (size_t)w0 * h->K : nullptr, d_R ? d_R + (size_t)w0 * h->m * h->m * 2 : nullptr,
-                             d_ev ? d_ev + (size_t)w0 * h->m : nullptr, s_scan, tev);
+                             d_ev ? d_ev + (size_t)w0 * h->m : nullptr, st, tev);
         if (rc) return rc;
-        CU(h, cudaEventRecord(ws.scan_done, s_scan));
+        CU(h, cudaEventRecord(ws.scan_done, st));
         ws.used = true;
-        last_slot = slot;
-        slot = pipe ? (slot + 1) % NSLOT : slot;
     }
-    if (pipe && last_slot >= 0) CU(h, cudaStreamWaitEvent(st, h->ws[last_slot].scan_done, 0));
     if (h->gather_G > 0) {
         const GatherFlags gf = make_gather_flags(h, true);
         if (gf.epoch) {
@@ -912,29 +867,12 @@ int music_b200_create(music_b200 **out, uint32_t m, uint32_t n, uint32_t nsample
                 CU(h, cudaMalloc(&h->table[i].na_max, sizeof(float)));
             }
         }
-        CU(h, cudaStreamCreateWithFlags(&h->s_cov, cudaStreamNonBlocking));
-        CU(h, cudaStreamCreateWithFlags(&h->s_scan, cudaStreamNonBlocking));
-        CU(h, cudaEventCreateWithFlags(&h->ev_in, cudaEventDisableTiming));
-        for (int i = 0; i < NSLOT; ++i) {
-            CU(h, cudaEventCreateWithFlags(&h->ws[i].cov_done, cudaEventDisableTiming));
-            CU(h, cudaEventCreateWithFlags(&h->ws[i].scan_done, cudaEventDisableTiming));
-        }
-        if (const char *e = getenv("MUSIC_B200_PIPE")) h->pipeline = atoi(e) != 0;
+        for (int i = 0; i < NSLOT; ++i) CU(h, cudaEventCreateWithFlags(&h->ws[i].scan_done, cudaEventDisableTiming));
         // scan kernels with M = 16 need 32 KiB dynamic smem (< 48 KiB default), nothing to opt in.
-        if (const char *e = getenv("MUSIC_B200_COV")) {  // kernel selection for A/B measurements
-            if (!strcmp(e, "ldg")) h->cov_tma_stages = 0;
-            else if (!strcmp(e, "tma4")) h->cov_tma_stages = 4;
-            else if (!strcmp(e, "tma6")) h->cov_tma_stages = 6;
-        }
-        if (const char *e = getenv("MUSIC_B200_SCAN")) h->scan_fast = strcmp(e, "general") != 0;
         if (const char *e = getenv("MUSIC_B200_FUSED")) h->fused = atoi(e) != 0;
-        if (const char *e = getenv("MUSIC_B200_COVN")) h->covn = atoi(e) != 0;
-        if (const char *e = getenv("MUSIC_B200_EIG")) h->eig_mode = !strcmp(e, "jacobi") ? 1 : !strcmp(e, "jacobi1") ? 2 : 0;
+        if (const char *e = getenv("MUSIC_B200_EIG")) h->eig_mode = !strcmp(e, "jacobi");
         if (const char *e = getenv("MUSIC_B200_PDL")) h->pdl = atoi(e) != 0;
-        if (const char *e = getenv("MUSIC_B200_DRAIN_NCH")) h->drain_nch = std::max(1, std::min((int)FZ_NCH, atoi(e)));
         if (const char *e = getenv("MUSIC_B200_FUSED_SPEC")) h->fused_spec = atoi(e) != 0;
-        if (const char *e = getenv("MUSIC_B200_EARLY_DRAIN")) h->early_drain = atoi(e) != 0;
-        if (const char *e = getenv("MUSIC_B200_IDLE_NS")) h->idle_ns = (unsigned)std::max(0, atoi(e));
         if (const char *e = getenv("MUSIC_B200_MMA_FIN")) h->mma_fin_max = std::max(-1, std::min(8, atoi(e)));
         CU(h, cudaFuncSetAttribute(covN_tma_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CN_SMEM));
         CU(h, cudaFuncSetAttribute(covN_tma_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)CN_SMEM));
@@ -953,8 +891,7 @@ int music_b200_create(music_b200 **out, uint32_t m, uint32_t n, uint32_t nsample
         CU(h, cudaFuncSetAttribute(music4_fused_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FZ_SMEM));
         CU(h, cudaFuncSetAttribute(music4_fused_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FZ_SMEM));
         CU(h, cudaFuncSetAttribute(music4_fused_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FZ_SMEM));
-        CU(h, cudaFuncSetAttribute(cov4_tma_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, 1024 + COV_WARPS * 6 * COV_CHUNK));
-        CU(h, cudaFuncSetAttribute(cov4_tma_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 1024 + COV_WARPS * 4 * COV_CHUNK));
+        CU(h, cudaFuncSetAttribute(cov4_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)COV_SMEM));
         return upload_table(h, 0, table_c64, h->streams[0]);
     };
     rc = init();
@@ -1010,7 +947,7 @@ int music_b200_process_planar_device(music_b200 *h, const float *const *d_stream
     std::lock_guard<std::mutex> g(h->mutex);
     CU(h, cudaSetDevice(h->device));
     return enqueue_device(h, nullptr, nwindows, d_angles, d_levels, d_spectrum, d_bins, nullptr, nullptr, nullptr,
-                          static_cast<cudaStream_t>(stream), 0, false, &S, hop);
+                          static_cast<cudaStream_t>(stream), 0, &S, hop);
 }
 
 int music_b200_process_planar_host(music_b200 *h, const float *const *streams, uint32_t hop, uint32_t nwindows,
@@ -1056,7 +993,7 @@ int music_b200_process_planar_host(music_b200 *h, const float *const *streams, u
         }
         if (rc) break;
         rc = enqueue_device(h, nullptr, W, h->d_ang[s], h->d_lvl[s], spectrum ? h->d_spec[s] : nullptr, h->d_bins[s],
-                            nullptr, nullptr, nullptr, st, s, false, &S, hop);
+                            nullptr, nullptr, nullptr, st, s, &S, hop);
         if (rc) break;
         rc = download_host_slot(h, s, w0, W, levels != nullptr, bins != nullptr, st);
         if (rc) break;
@@ -1253,7 +1190,7 @@ int music_b200_process_device_ex(music_b200 *h, const float *d_in_c64, uint32_t 
         ++h->gather_epoch;
     }
     return enqueue_device(h, d_in_c64, nwindows, d_angles, d_levels, d_spectrum, d_bins, d_P64, d_R, d_eigvals,
-                          static_cast<cudaStream_t>(stream), 0, true);
+                          static_cast<cudaStream_t>(stream), 0);
 }
 
 int music_b200_process_device(music_b200 *h, const float *d_in_c64, uint32_t nwindows, float *d_angles,
@@ -1321,7 +1258,7 @@ int music_b200_process_host(music_b200 *h, const float *in_c64, uint32_t nwindow
             {
                 NvtxRange r("music_b200: kernels");
                 rc = enqueue_device(c, c->d_in[s], W, c->d_ang[s], c->d_lvl[s], spectrum ? c->d_spec[s] : nullptr, c->d_bins[s],
-                                    nullptr, nullptr, nullptr, st, s, false);
+                                    nullptr, nullptr, nullptr, st, s);
                 if (rc && c != h) fail(h, rc, "%s", std::string(c->error).c_str());
                 if (rc) break;
             }
@@ -1498,7 +1435,7 @@ int music_b200_process_device_sharded(music_b200 *h, const float *const *d_in_c6
         c->gather_rank = l;
         for (int p = 0; p < G; ++p) { c->peer_bins[p] = d_bins_all ? d_bins_all[p] : nullptr; c->peer_flags[p] = nullptr; }
         rc = enqueue_device(c, d_in_c64[l], Wl, d_angles[l], d_levels ? d_levels[l] : nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
-                            streams ? static_cast<cudaStream_t>(streams[l]) : nullptr, 0, false);
+                            streams ? static_cast<cudaStream_t>(streams[l]) : nullptr, 0);
         c->gather_G = 0;
         if (rc) fail(h, rc, "%s", std::string(c->error).c_str());
     }
@@ -1523,12 +1460,8 @@ void music_b200_destroy(music_b200 *h)
     for (int i = 0; i < NSLOT; ++i) {
         Workspace &ws = h->ws[i];
         cudaFree(ws.R); cudaFree(ws.ev); cudaFree(ws.Vt); cudaFree(ws.P64);
-        if (ws.cov_done) cudaEventDestroy(ws.cov_done);
         if (ws.scan_done) cudaEventDestroy(ws.scan_done);
     }
-    if (h->s_cov) cudaStreamDestroy(h->s_cov);
-    if (h->s_scan) cudaStreamDestroy(h->s_scan);
-    if (h->ev_in) cudaEventDestroy(h->ev_in);
     cudaFree(h->fused_trace);
     cudaFree(h->f8_stats);
     cudaFree(h->work_ctr);

@@ -184,7 +184,7 @@ __device__ __forceinline__ bool eig8_principal_warp(double2 *S, double2 *Vt, con
 
 __global__ void __launch_bounds__(F8_WARPS * 32, 1)
 music8_fused_kernel(const __grid_constant__ CUtensorMap tm, const double *__restrict__ soa, int W, int N, int K, const PeakOut out,
-                    unsigned *__restrict__ work_ctr, const GatherFlags gather_flags, const int eig_mode /* 0: squaring, 1: Jacobi */,
+                    unsigned *__restrict__ work_ctr, const GatherFlags gather_flags, const bool eig_mode /* false: squaring; true: Jacobi */,
                     unsigned *__restrict__ stats /* optional [2]: windows solved by squaring / by Jacobi */)
 {
     const unsigned long long tm_addr = reinterpret_cast<unsigned long long>(&tm);
@@ -344,7 +344,7 @@ music8_fused_kernel(const __grid_constant__ CUtensorMap tm, const double *__rest
         // eigenvectors of this window -> batch slot nb
         double2 *Vt = Vb + 64 * nb;
         bool solved = false;
-        if (eig_mode == 0) solved = eig8_principal_warp(Rw, Vt, lane);
+        if (!eig_mode) solved = eig8_principal_warp(Rw, Vt, lane);
         if (solved) {
             ++n_sq;
         } else {

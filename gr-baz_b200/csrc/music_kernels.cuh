@@ -167,10 +167,12 @@ __global__ void __launch_bounds__(256) cov_tile_kernel(const float *__restrict__
 // needs a barrier.  The ring runs across window boundaries, i.e. the next window's first
 // chunks are already in flight during the warp-shuffle reduction of the current one.
 // Per snapshot and lane: 2 LDS.128, 8 F2F (exact widening), 32 DFMA into 16 accumulators
-// (Hermitian half of x x^H).  Bytes in flight per SM = 8 warps x (STAGES-1) x 4 KiB.
+// (Hermitian half of x x^H).  Bytes in flight per SM = 8 warps x (COV_STAGES-1) x 4 KiB.
 // ------------------------------------------------------------------------------------------
 constexpr int COV_CHUNK = 4096;  // bytes per stage = 128 snapshots of 4 antennas
 constexpr int COV_WARPS = 8;
+constexpr int COV_STAGES = 6;
+constexpr size_t COV_SMEM = 1024 + (size_t)COV_WARPS * COV_STAGES * COV_CHUNK;  // barriers + rings
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count)
@@ -251,14 +253,13 @@ __device__ __forceinline__ void cov4_accumulate(double (&acc)[16], const float4 
     acc[14] = fma(r2, r3, fma(i2, i3, acc[14]));  acc[15] = fma(i2, r3, fma(-r2, i3, acc[15]));  // 23
 }
 
-template <int STAGES>
 __global__ void __launch_bounds__(COV_WARPS * 32, 1) cov4_tma_kernel(const float *__restrict__ in, double *__restrict__ R,
                                                                      int W, int N)
 {
     extern __shared__ __align__(128) unsigned char cov_smem[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    uint64_t *bars = reinterpret_cast<uint64_t *>(cov_smem) + warp * STAGES;  // first 1 KiB: barriers
-    unsigned char *ring = cov_smem + 1024 + (size_t)warp * STAGES * COV_CHUNK;
+    uint64_t *bars = reinterpret_cast<uint64_t *>(cov_smem) + warp * COV_STAGES;  // first 1 KiB: barriers
+    unsigned char *ring = cov_smem + 1024 + (size_t)warp * COV_STAGES * COV_CHUNK;
     const uint32_t bar0 = smem_u32(bars), ring0 = smem_u32(ring);
 
     const int gw = blockIdx.x * COV_WARPS + warp, total_warps = gridDim.x * COV_WARPS;
@@ -269,7 +270,7 @@ __global__ void __launch_bounds__(COV_WARPS * 32, 1) cov4_tma_kernel(const float
     const unsigned char *src0 = reinterpret_cast<const unsigned char *>(in);
 
     if (lane == 0) {
-        for (int s = 0; s < STAGES; ++s) mbar_init(bar0 + 8 * s, 1);
+        for (int s = 0; s < COV_STAGES; ++s) mbar_init(bar0 + 8 * s, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     }
@@ -280,13 +281,13 @@ __global__ void __launch_bounds__(COV_WARPS * 32, 1) cov4_tma_kernel(const float
         const int j = (int)(c / cpw), q = (int)(c % cpw);
         const size_t off = (size_t)q * COV_CHUNK;
         const uint32_t bytes = (uint32_t)min((size_t)COV_CHUNK, win_bytes - off);
-        const int slot = (int)(c % STAGES);
+        const int slot = (int)(c % COV_STAGES);
         const unsigned char *src = src0 + ((size_t)gw + (size_t)j * total_warps) * win_bytes + off;
         mbar_expect_tx(bar0 + 8 * slot, bytes);
         bulk_g2s_hint(ring0 + slot * COV_CHUNK, src, bytes, bar0 + 8 * slot, pol_stream);
     };
     if (lane == 0)
-        for (long long c = 0; c < total && c < STAGES; ++c) issue(c);
+        for (long long c = 0; c < total && c < COV_STAGES; ++c) issue(c);
 
     double acc[16];
 #pragma unroll
@@ -312,8 +313,8 @@ __global__ void __launch_bounds__(COV_WARPS * 32, 1) cov4_tma_kernel(const float
             for (int s = lane; s < nsnap; s += 32) cov4_accumulate(acc, buf[2 * s], buf[2 * s + 1]);
         }
         __syncwarp();  // every lane is done reading the slot -> it may be refilled
-        if (lane == 0 && c + STAGES < total) issue(c + STAGES);
-        if (++slot == STAGES) { slot = 0; parity ^= 1; }
+        if (lane == 0 && c + COV_STAGES < total) issue(c + COV_STAGES);
+        if (++slot == COV_STAGES) { slot = 0; parity ^= 1; }
         if (++q == cpw) {
             q = 0;
 #pragma unroll

@@ -268,8 +268,8 @@ def test_fused_kernel_matches_unfused_path_on_every_window(monkeypatch, eig, mma
                      drain workers, dynamic tickets change nothing);
       eig = power  : (default) principal eigenvector by squaring instead of Jacobi: an independent algorithm, so the
                      bins must be identical and the levels agree to 1e-9 (P is conditioned ~4000x, both are ~1e-12).
-      mma_fin      : 2 = default hand-over to the drain workers, -1 = fp64 drain workers only, 8 = tensor-core passes
-                     to the very end (the round-1 behaviour)."""
+      mma_fin      : 2 = hand-over to the drain workers one covariance warp earlier than the default (3), -1 = fp64
+                     drain workers only, 8 = tensor-core passes to the very end (the round-1 behaviour)."""
     cfg = synth.config(2)
     table = helpers.table_for(cfg)
     dev = torch.device("cuda:0")

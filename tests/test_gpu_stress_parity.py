@@ -29,9 +29,9 @@ P_RTOL = 1e-5
 TIE_ALLOWANCE = 2
 SCAN_B = 8
 MAX_SUB_M16_K36000 = 1352  # max_sub_windows(): 384 MiB / (16*16*2*8*2 + 16*8 + 36000*8) bytes, rounded down to SCAN_B
+MAX_SUB_M16 = 48392  # the same without fp64 strengths in the workspace (d_P64 given): 384 MiB / (16*16*2*8*2 + 16*8), rounded down
 DEV = torch.device("cuda:0")
-ENV_KEYS = ("MUSIC_B200_FUSED", "MUSIC_B200_FUSED_SPEC", "MUSIC_B200_EIG", "MUSIC_B200_TRACE", "MUSIC_B200_MMA_FIN",
-            "MUSIC_B200_PIPE", "MUSIC_B200_SCAN")
+ENV_KEYS = ("MUSIC_B200_FUSED", "MUSIC_B200_FUSED_SPEC", "MUSIC_B200_EIG", "MUSIC_B200_TRACE", "MUSIC_B200_MMA_FIN")
 
 
 def make_block(monkeypatch, cfg, table, env=None):
@@ -323,8 +323,8 @@ def test_fused_and_unfused_agree_on_families(monkeypatch, m):
         assert helpers.rel_err(outs["default"]["levels"], u["levels"]) <= 1e-9, key
 
 
-def _check_every_window_against_single_runs(blk, cfg, table, x, got, spectrum, p64, internals, sample):
-    for w in range(x.shape[0]):
+def _check_every_window_against_single_runs(blk, cfg, table, x, got, spectrum, p64, internals, sample, windows=None):
+    for w in (range(x.shape[0]) if windows is None else windows):
         one = run_device(blk, cfg, x[w:w + 1], spectrum=spectrum, p64=p64, internals=internals)
         for f in ("bins", "angles", "levels", "spectrum", "P", "R", "eigvals"):
             if f in one:
@@ -333,20 +333,21 @@ def _check_every_window_against_single_runs(blk, cfg, table, x, got, spectrum, p
     assert_matches_oracle({k: v[sample] for k, v in got.items() if k != "launches"}, ref, x[sample], cfg["resolution"])
 
 
-def test_pipelined_sub_batches_with_every_output(monkeypatch):
-    """2 049 windows, MUSIC_B200_PIPE=1: two sub-batches on two streams and two workspace slots, with d_spec, d_P64, d_R
-    and d_eigvals requested; every window against a single-window call of the same handle, a sample against the oracle"""
-    cfg = synth.config(1, snapshots=64, resolution=449)
+def test_sub_batches_with_every_output(monkeypatch):
+    """M = 16, n = 2: MAX_SUB_M16 + 5 windows, two sub-batches through one workspace slot, with d_spec, d_P64, d_R and
+    d_eigvals requested; windows on both sides of the boundary and a stride sample against single-window calls of the
+    same handle, the sample against the oracle"""
+    cfg = synth.config(5, snapshots=128, resolution=360)
     table = helpers.table_for(cfg)
-    W = 2049
+    W = MAX_SUB_M16 + 5
     x = synth.gen_windows_numpy(cfg, 4049, 0, W)
-    blk = make_block(monkeypatch, cfg, table, {"MUSIC_B200_PIPE": "1"})
+    blk = make_block(monkeypatch, cfg, table)
     got = run_device(blk, cfg, x, spectrum=True, p64=True, internals=True)
-    assert got["launches"] == 2 * unfused_launches(4, 1, 64)  # 2 sub-batches of 1032 / 1017 windows
-    sample = np.unique(np.concatenate([np.arange(0, W, 97), [1031, 1032, 1033, W - 1]]))
-    _check_every_window_against_single_runs(blk, cfg, table, x, got, True, True, True, sample)
+    assert got["launches"] == 2 * unfused_launches(16, 2, 128)
+    sample = np.unique(np.concatenate([np.arange(0, W, 4999), [MAX_SUB_M16 - 1, MAX_SUB_M16, MAX_SUB_M16 + 1, W - 1]]))
+    _check_every_window_against_single_runs(blk, cfg, table, x, got, True, True, True, sample, windows=sample)
     for w in sample:
-        R = mo.covariance(x[w], 4)
+        R = mo.covariance(x[w], 16)
         assert np.max(np.abs(got["R"][w] - R)) <= 1e-12 * np.max(np.abs(R))
         assert np.max(np.abs(got["eigvals"][w] - np.linalg.eigvalsh(R))) <= 1e-11 * np.max(np.abs(R))
     blk.close()
